@@ -9,8 +9,7 @@ collective on the solve path; NCCL only for the barrier and the max-over-ranks).
 sharded over the N GPUs: strong scaling).
 
   value      device-resident throughput: inputs in HBM, rotating over input sets larger than L2; the timed
-             region is run `blocks` times (each EXACTLY --steps launches, barrier + synchronize on both sides)
-             and `value` is the median block, max over ranks (`block_ms` lists them all)
+             region is EXACTLY --steps launches (barrier + synchronize on both sides), max over ranks
   e2e        same metric through the public API LQRStep(...)(x_init,C,c,F,f) with the inputs in
              pinned HOST memory: H2D of the step's inputs and D2H of its results inside the timing
   roofline   algorithmic bytes per launch / kernel time  vs the measured HBM copy peak
@@ -39,6 +38,7 @@ import warnings
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOADS = {
@@ -140,7 +140,7 @@ class RawStepper:
         from mpc.pytorch_b200._lib import Dims, Params, ptr
         dev = inp["C"].device
         self.out = dict(new_x=torch.empty(T, B, n, device=dev), new_u=torch.empty(T, B, m, device=dev),
-                        costs=torch.empty(B, device=dev), fdn=torch.empty(B, device=dev),
+                        costs=torch.empty(B, device=dev), full_du_norm=torch.empty(B, device=dev),
                         alphas=torch.empty(B, device=dev))
         kind = 0 if bounds is None and tensor_bounds is None else (2 if tensor_bounds is not None else 1)
         self.dims = Dims(B=B, T=T, n=n, m=m, F_T=T - 1, has_f=1, bounds_kind=kind, has_zero_mask=0,
@@ -156,7 +156,7 @@ class RawStepper:
             self.ks = torch.empty(T, B, m, device=dev)
         self.args = [ctypes.byref(self.dims), ctypes.byref(self.params), ptr(inp["C"]), ptr(inp["c"]),
                      ptr(inp["F"]), ptr(inp["f"]), ptr(inp["x_init"]), ptr(inp["cur_x"]), ptr(inp["cur_u"]),
-                     ptr(lo), ptr(hi), None, ptr(o["new_x"]), ptr(o["new_u"]), ptr(o["costs"]), ptr(o["fdn"]),
+                     ptr(lo), ptr(hi), None, ptr(o["new_x"]), ptr(o["new_u"]), ptr(o["costs"]), ptr(o["full_du_norm"]),
                      ptr(o["alphas"]), None, None, None, None, ptr(self.Ks), ptr(self.ks), None]
         self.keep = (inp, lo, hi)
 
@@ -196,6 +196,22 @@ class RawAdjoint:
         rc = self.fn(*self.args)
         if rc != 0:
             raise RuntimeError(f"mpcb200_lqr_adjoint_f32 -> {rc}")
+
+
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def dump_outputs(out, B, path):
+    """Writes the arrays one step call returns (new_x, new_u [T,B,.]; costs, full_du_norm, alphas [B]) as float32
+    `path/<name>.npy`.  Outputs larger than DUMP_MAX_BYTES are cut to a fixed, seeded sample of the problems (the
+    same in every run, kept in batch order), so that the dumps of two builds compare output for output."""
+    per_problem = sum(v.numel() // B * v.element_size() for v in out.values())
+    keep = min(B, (DUMP_MAX_BYTES - 4096) // per_problem)       # 4 kB left for the .npy headers
+    idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        v = v.index_select(0 if v.dim() == 1 else 1, idx.to(v.device))
+        np.save(os.path.join(path, name + ".npy"), v.cpu().numpy())
 
 
 # --------------------------------------------------------------------------------------------- CPU arms
@@ -377,14 +393,19 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="config3", choices=sorted(WORKLOADS))
-    ap.add_argument("--blocks", type=int, default=5, help="timed blocks of --steps launches (value = median block)")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary figures (adjoint, box, config 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MB)")
     a = ap.parse_args()
-    # watchdog: a hung bench must not eat the box; dumps all Python stacks and exits
-    faulthandler.dump_traceback_later(int(os.environ.get("BENCH_WATCHDOG_S", "900")), exit=True)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or world > 1):
+        ap.error("--dump-outputs writes the CUDA step's outputs of a single process (--impl b200, one rank)")
+    # watchdog: a hung bench must not eat the box; dumps all Python stacks and exits
+    faulthandler.dump_traceback_later(int(os.environ.get("BENCH_WATCHDOG_S", "900")), exit=True)
     cfg = dict(WORKLOADS[a.workload])
     T, n, m = cfg["T"], cfg["n"], cfg["m"]
     B = cfg["B"] if cfg["scaling"] == "weak" else cfg["B"] // max(1, a.gpus)      # problems per GPU
@@ -444,26 +465,23 @@ def main():
         torch.cuda.synchronize(dev)
     for w in range(a.warmup):
         steppers[w % n_sets](sh)
-    block_ms = []
-    launches = 0
-    for blk in range(max(1, a.blocks)):
-        barrier()
-        l0 = _lib.launch_count()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(stream)
-        for k in range(a.steps):
-            steppers[k % n_sets](sh)
-        e1.record(stream)
-        barrier()
-        launches = _lib.launch_count() - l0
-        t_ms = e0.elapsed_time(e1)
-        if world > 1:
-            tms = torch.tensor([t_ms], device=dev)
-            dist.all_reduce(tms, op=dist.ReduceOp.MAX)
-            t_ms = float(tms.item())
-        block_ms.append(t_ms)
-    ms = statistics.median(block_ms)
+    barrier()
+    l0 = _lib.launch_count()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record(stream)
+    for k in range(a.steps):
+        steppers[k % n_sets](sh)
+    e1.record(stream)
+    barrier()
+    launches = _lib.launch_count() - l0
+    ms = e0.elapsed_time(e1)
+    if world > 1:
+        tms = torch.tensor([ms], device=dev)
+        dist.all_reduce(tms, op=dist.ReduceOp.MAX)
+        ms = float(tms.item())
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs:
+        dump_outputs(steppers[(a.steps - 1) % n_sets].out, B, a.dump_outputs)
 
     # ---------------- e2e: public API, host buffers, copies inside the timed region
     # Two streams: the copy-in stream feeds double-buffered device inputs while the run stream solves the
@@ -510,7 +528,7 @@ def main():
             h_out[1].copy_(nu, non_blocking=True)
             h_out[2].copy_(costs, non_blocking=True)
 
-    e2e_steps = max(3, min(a.steps, 50 if a.workload == "config3" else 6))
+    e2e_steps = min(a.steps, 50 if a.workload == "config3" else 6)     # bounded: a config-5 step moves up to 5 GB over PCIe
     with torch.no_grad(), numa_local(dev):             # the submitting thread runs next to the GPU as well
         for k in range(3):
             e2e_step(k)
@@ -566,7 +584,6 @@ def main():
     out.update({
         "value": B * world * a.steps / (ms * 1e-3), "ms_per_step": ms / a.steps,
         "gpu_launches": int(launches), "clocks": clocks,
-        "blocks": len(block_ms), "block_ms": [round(x, 4) for x in block_ms],
         "e2e": {"value": B * world * e2e_steps / e2e_s, "unit": "solves/s",
                 "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h), "steps": e2e_steps,
                 "h2d_gbs_achieved": round(h2d * e2e_steps / e2e_s / 1e9, 2), "h2d_gbs_measured_peak": round(pcie, 2),
@@ -583,7 +600,7 @@ def main():
                      "peak_source": peak_src, "kernel": f"lqr_step<float,{n},{m}>",
                      "algorithmic_bytes_per_launch": bps * B, "bytes_per_solve": bps},
         "timing": {"l2_policy": f"rotating {n_sets} input sets ({n_sets * bps * B / 1e6:.0f} MB > 126 MB L2)",
-                   "preheat_s": preheat, "value_is": f"median of {len(block_ms)} blocks of {a.steps} launches, max over ranks"},
+                   "preheat_s": preheat, "value_is": f"one timed window of {a.steps} launches, max over ranks"},
     })
     if a.workload == "config5":
         fl = flops_per_solve(T, n, m)

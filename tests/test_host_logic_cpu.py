@@ -17,6 +17,34 @@ def test_bytes_per_solve_matches_survey_table():
     assert bench.bytes_per_solve(50, 16, 4) == 157928
 
 
+def test_bench_dump_outputs_whole_batch_or_fixed_sample(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: the whole batch while it fits the size limit, else the same seeded sample of
+    problems in every run, taken from every output along its batch axis, within the limit."""
+    import numpy as np
+    import bench
+    T, B, n, m = 4, 64, 3, 2
+    g = torch.Generator().manual_seed(1)
+    out = dict(new_x=torch.randn(T, B, n, generator=g), new_u=torch.randn(T, B, m, generator=g),
+               costs=torch.arange(B, dtype=torch.float32), full_du_norm=torch.randn(B, generator=g),
+               alphas=torch.rand(B, generator=g))
+    bench.dump_outputs(out, B, str(tmp_path / "all"))
+    for k, v in out.items():
+        got = np.load(tmp_path / "all" / f"{k}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, v.numpy()), k
+    limit = 20 * (T * (n + m) + 3) * 4 + 4096               # room for 20 of the 64 problems
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", limit)
+    for d in ("a", "b"):
+        bench.dump_outputs(out, B, str(tmp_path / d))
+    idx = np.load(tmp_path / "a" / "costs.npy").astype(np.int64)    # costs[b] == b names the sampled problems
+    assert len(idx) == 20 and np.all(np.diff(idx) > 0)
+    total = 0
+    for k, v in out.items():
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert np.array_equal(a, b) and np.array_equal(a, v.numpy()[idx] if v.dim() == 1 else v.numpy()[:, idx]), k
+        total += (tmp_path / "a" / f"{k}.npy").stat().st_size
+    assert total <= limit
+
+
 @pytest.mark.parametrize("shape,bounds", [((3, 3), 0.3), ((6, 1), None), ((5, 3), "tensor")])
 def test_padding_embedding_is_exact(shape, bounds):
     """step._Pad: the padded problem solved by the ORACLE equals the original problem (so a padded
